@@ -182,9 +182,11 @@ def run_reference(args, rank, world):
     print(json.dumps(line))
 
 
-def measure_workload(ms, torch, workload, B, rank, local_rank, args, steps, warmup, min_it=ITERS, max_it=ITERS, e2e=True, profile=True, flush=None, barrier=None):
+def measure_workload(ms, torch, workload, B, rank, local_rank, args, steps, warmup, min_it=ITERS, max_it=ITERS, e2e=True, profile=True, flush=None, barrier=None,
+                     keep_outputs=False):
     """Device-resident timing (CUDA events on the launching stream, L2 flushed between steps), the end-to-end leg through mb2_set_targets +
-    mb2_solver_solve with pinned host buffers, and one profiling solve (events around every launch + in-kernel phase cycles)."""
+    mb2_solver_solve with pinned host buffers, and one profiling solve (events around every launch + in-kernel phase cycles).
+    keep_outputs: out["outputs"] holds what the last timed step returned to its caller (solved parameters + per-instance results)."""
     ch, efs, theta0, _ = make_problem(workload, B, seed_offset=1000 * rank)  # each rank owns a different shard
     n = ch.num_params
     fn = ms.SkeletonSolverFunction(ch, B, efs, device=local_rank)
@@ -217,6 +219,8 @@ def measure_workload(ms, torch, workload, B, rank, local_rank, args, steps, warm
     res = solver.get_results()
     out = {"ch": ch, "efs": efs, "n": n, "B": B, "solver": solver, "fn": fn, "total_ms": total_ms, "its_per_step": int(res["iterations"].sum()),
            "err_sum": float(res["errors"].sum()), "launches": solver.get_counters()[1], "status_bad": int((res["status"] != 0).sum())}
+    if keep_outputs:  # before the profiling and end-to-end solves below overwrite theta_dev
+        out["outputs"] = {"params": theta_dev.cpu().numpy(), **res}
     if profile:
         solver.set_profiling(1)  # events around the production kernels: the per-kernel times
         device_step()
@@ -263,6 +267,25 @@ def measure_workload(ms, torch, workload, B, rank, local_rank, args, steps, warm
         out["h2d"] = int(theta0_pin.numel() * 4 + sum(tp.numel() * 4 for tp in target_pins))
         out["d2h"] = int(theta0_pin.numel() * 4 + B * (8 + 4 + 4))
     return out
+
+
+DUMP_LIMIT_BYTES = 64 * 2 ** 20
+
+
+def dump_outputs(directory, outputs, prefix=""):
+    """--dump-outputs: what the last timed step returned, one row per instance, as <directory>/<prefix><name>.npy (parameters float32, per-instance
+    results float64) so that two builds can be compared output for output. Above DUMP_LIMIT_BYTES in all a fixed seeded sample of the
+    instances is written; instance.npy always lists the instances written."""
+    arrays = {"params": outputs["params"].astype(np.float32), "errors": outputs["errors"].astype(np.float64),
+              "iterations": outputs["iterations"].astype(np.float64), "status": outputs["status"].astype(np.float64)}
+    B = arrays["params"].shape[0]
+    row_bytes = sum(a[0].nbytes for a in arrays.values()) + 8  # + the instance index
+    keep = min(B, (DUMP_LIMIT_BYTES - 4096) // row_bytes)  # 4096: the .npy headers
+    idx = np.arange(B) if keep == B else np.sort(np.random.default_rng(0).choice(B, keep, replace=False))
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, prefix + "instance.npy"), idx.astype(np.float64))
+    for name, a in arrays.items():
+        np.save(os.path.join(directory, prefix + name + ".npy"), a[idx])
 
 
 def kernel_report(m, peaks, workload):
@@ -446,7 +469,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--clock-poll-ms", type=float, default=25.0, help="NVML clock / throttle-reason sampling period during the timed regions")
     ap.add_argument("--no-extras", action="store_true", help="skip the other workloads measured in the same run (cfg2, cfg4, cfg5, convergence mode)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the last step's solved parameters and per-instance results to "
+                    "DIR/<name>.npy (DIR/rank<r>_<name>.npy with several ranks); the inputs are seeded, so runs with the same arguments are comparable")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.sharded > 0 or args.workload == "cfg5"):
+        ap.error("--dump-outputs covers the device-resident path of cfg2, cfg3-shard and cfg4")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
@@ -497,8 +526,11 @@ def main():
 
     sampler = ClockSampler(local_rank, args.clock_poll_ms * 1e-3)
     sampler.start()
-    m = measure_workload(ms, torch, args.workload, B, rank, local_rank, args, args.steps, args.warmup, flush=flush, barrier=barrier)
+    m = measure_workload(ms, torch, args.workload, B, rank, local_rank, args, args.steps, args.warmup, flush=flush, barrier=barrier,
+                         keep_outputs=bool(args.dump_outputs))
     clocks = sampler.stop()  # sampled across the device-resident and the end-to-end timed regions
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, m.pop("outputs"), prefix=f"rank{rank}_" if world > 1 else "")
     # the one collective of the path: aggregate iterations / residual norm (SUM) and elapsed device time (MAX over ranks)
     from momentum_b200.distributed import aggregate_solve_stats
 

@@ -7,14 +7,16 @@ from __future__ import annotations
 
 import ctypes as C
 import os
+import shutil
 import subprocess
+import sys
+import tempfile
 from typing import Optional, Sequence
 
 import numpy as np
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIB_PATH = os.path.join(_HERE, "liboracle.so")
-_NATIVE_PATH = os.path.join(_HERE, "liboracle_native.so")  # timing arm only, built on the machine that runs it (oracle/Makefile)
 _lib = None
 _native = None
 
@@ -31,16 +33,21 @@ def build(force: bool = False) -> str:
 
 def native_lib():
     """The -march=native / fast-math build for bench.py's CPU arm. Always rebuilt by the process that times it (a copy built on
-    another host may use instructions this one lacks); falls back to the portable checker build if the compile fails."""
+    another host may use instructions this one lacks), into a temporary directory so that the source tree is never written; falls
+    back to the portable checker build if the compile fails."""
     global _native
     if _native is None:
+        tmp = tempfile.mkdtemp(prefix="oracle_native_")
         try:
-            subprocess.check_call(["make", "-C", _HERE, "-s", "-B", "native"])
-            _native = _bind(C.CDLL(_NATIVE_PATH))
+            path = os.path.join(tmp, "liboracle_native.so")
+            subprocess.check_call(["make", "-C", _HERE, "-s", "-B", "native", f"NATIVE_OUT={path}"])
+            _native = _bind(C.CDLL(path))  # the mapping outlives the file, so the directory can go at once
             _native.is_native = True
         except Exception as e:  # noqa: BLE001
-            print(f"[oracle] native build unavailable ({e}); timing the portable build", flush=True)
+            print(f"[oracle] native build unavailable ({e}); timing the portable build", file=sys.stderr, flush=True)
             _native = lib()
+        finally:
+            shutil.rmtree(tmp, ignore_errors=True)
     return _native
 
 
